@@ -215,7 +215,7 @@ def cpu_decode_pass(fs, threads, buf=None):
         buf = np.zeros(fs.D + 64, dtype=np.uint8)   # pre-touched: page faults stay out of the timing
     t0 = time.perf_counter()
     out, sizes = O.bulk_decode(fs.comp, fs.src_off, fs.src_size, fs.out_off, fs.out_size, raw_dict=rd, nthreads=threads, out=buf)
-    return time.perf_counter() - t0, out
+    return time.perf_counter() - t0, out, sizes
 
 
 def libzstd_one_core(fs, budget_s=2.0):
@@ -246,12 +246,36 @@ def cpu_baseline(fs, threads=None, passes=2):
     cpu_decode_pass(fs, threads, buf)   # warm-up (page tables, thread stacks)
     best, out = None, None
     for _ in range(passes):
-        dt, out = cpu_decode_pass(fs, threads, buf)
+        dt, out, _ = cpu_decode_pass(fs, threads, buf)
         best = dt if best is None else min(best, dt)
     assert np.array_equal(out[:fs.D], fs.plain), "CPU port output differs from the generator's plaintext"
     return {"value": fs.D / best / GB, "unit": "GB/s", "cores": threads, "kind": "port",
             "sample": f"all {fs.nframes} frames ({fs.D / 2**20:.0f} MiB) of the same workload, one FrameDecoder per thread, best of {passes} passes after a warm-up",
             "one_core_GBps": sub.D / one / GB, "libzstd_1.5.5_one_core_GBps": libzstd_one_core(fs)}
+
+
+DUMP_BYTES = 1 << 21    # --dump-outputs: decoded bytes kept (float32 value + float64 position: 24 MiB)
+DUMP_FRAMES = 1 << 19   # and frames kept (five float64 arrays: at most 20 MiB)
+
+
+def sample_index(n, cap):
+    """Sorted positions of a fixed, seeded sample of `cap` of `n` items (all of them when n <= cap)."""
+    if n <= cap:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.Generator(np.random.PCG64(0xD0D0)).choice(n, cap, replace=False, shuffle=False))
+
+
+def dump_outputs(path, out_index, out_values, frames):
+    """--dump-outputs: write what the timed path returned in its last step as float32 / float64 .npy files, so that two builds
+    run with the same arguments can be compared output for output.  output.npy holds the decoded bytes at the positions in
+    output_index.npy (offsets into the concatenated output of all frames); frame_<field>.npy holds the per-frame results
+    {field: array over all frames} of the frames listed in frame_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    fi = sample_index(len(next(iter(frames.values()))), DUMP_FRAMES)
+    arrays = {"output_index": out_index.astype(np.float64), "output": np.asarray(out_values).astype(np.float32), "frame_index": fi.astype(np.float64)}
+    arrays.update({"frame_" + k: np.asarray(v)[fi].astype(np.float64) for k, v in frames.items()})
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def run_reference(args):
@@ -267,10 +291,13 @@ def run_reference(args):
     warm = max(1, min(args.warmup, 3))
     times = []
     for i in range(warm + steps):
-        dt, out = cpu_decode_pass(fs, threads, buf)
+        dt, out, sizes = cpu_decode_pass(fs, threads, buf)
         if i >= warm:
             times.append(dt)
     assert np.array_equal(out[:fs.D], fs.plain), "CPU port output differs from the generator's plaintext"
+    if args.dump_outputs:
+        bi = sample_index(fs.D, DUMP_BYTES)
+        dump_outputs(args.dump_outputs, bi, out[bi], {"out_size": sizes})
     dt = sum(times)
     val = fs.D * steps / dt / GB
     line = {"impl": "reference", "metric": "decompressed_GBps", "value": val, "unit": "GB/s", "n_gpus": args.gpus, "steps": steps,
@@ -315,7 +342,11 @@ def main():
     ap.add_argument("--c5-frames", type=int, default=100000)
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(a seeded sample of the decoded bytes and the per-frame results; with N > 1, those of rank 0)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.steps_given = args.steps is not None
     if args.steps is None:
         args.steps = 50 if args.config != "c2a" else 3   # one chained 1 GiB frame is a serial chain of 8192 blocks: seconds per pass
@@ -388,7 +419,12 @@ def main():
         launches = ctx.kernel_launches() - launches0
         res = batch.finish()
         assert (res["status"] == 0).all(), "a frame failed inside the timed region: %r" % (res[res["status"] != 0][:3],)
-        out = {"fs": fs, "batch": batch, "d_out": d_out, "bit_exact": bit_exact, "ms": ms, "launches": launches, "clocks": clocks, "info": batch.info(),
+        last = None
+        if args.dump_outputs:   # what the last timed pass left in d_out, before any later pass reuses it
+            bi = sample_index(D, DUMP_BYTES)
+            last = (bi, d_out[torch.from_numpy(bi).to(d_out.device)].cpu().numpy(),
+                    {k: res[k] for k in ("status", "out_size", "bytes_read", "calculated_checksum")})
+        out = {"last_step": last, "fs": fs, "batch": batch, "d_out": d_out, "bit_exact": bit_exact, "ms": ms, "launches": launches, "clocks": clocks, "info": batch.info(),
                "sched": batch.debug_sched()}
         # the same passes without the checksum stage (what round 1 timed)
         ctx.set_flags(0)
@@ -485,6 +521,8 @@ def main():
             line["cpu_affinity"] = numa
         if not args.skip_cpu and world == 1:   # the CPU baseline is a single-GPU-run companion (rank 0, N = 1 only)
             line["cpu_baseline"] = cpu_baseline(fs_all)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *M["last_step"])
         print(json.dumps(line))
     barrier()
     if world > 1:

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Generate tests/golden/ from the reference's own golden vectors (run in the build container only).
+"""Generate tests/golden/ from the reference's own golden vectors.  usage: make_golden.py <zstd-rs checkout>
 
 The reference (KillingSpark/zstd-rs @ eb7e03cc) is Rust and cannot be executed here, so the vectors are the
 ones its own tests assert on (SURVEY.md section 8c):
@@ -8,12 +8,14 @@ ones its own tests assert on (SURVEY.md section 8c):
   * ruzstd/test_fixtures/*.zst                    (tests/mod.rs:576-741; plaintexts generated in code)
   * ruzstd/fuzz/artifacts/*/*                     (tests/fuzz_regressions.rs, fse/mod.rs, huff0/mod.rs)
 Compressed inputs are copied verbatim (they are test DATA, not source); expected plaintexts are recorded as
-size + SHA-256 + XXH64-low32 in manifest.json so the repo stays small.  /root/reference does not exist on
-the GPU box, so every test reads tests/golden/ only.
+size + SHA-256 + XXH64-low32 in manifest.json so the repo stays small, and byte windows of every decode-corpus
+original (first and last 64 bytes, four seeded 32-byte windows in between) go to decodecorpus_originals.npz.
+Every test reads tests/golden/ only; the reference checkout is needed to regenerate it, not to run the tests.
 """
 import hashlib, json, os, shutil, sys
 
-REF = "/root/reference/ruzstd"
+import numpy as np
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 
@@ -22,11 +24,22 @@ def sha(b):
     return hashlib.sha256(b).hexdigest()
 
 
-def main():
+def original_windows(orig, rng):
+    """(offset, length) of the stored windows of one original: all of it when short, else head, tail and 4 seeded windows."""
+    if len(orig) <= 256:
+        return [(0, len(orig))]
+    mid = sorted(int(x) for x in rng.integers(64, len(orig) - 96, 4))
+    return [(0, 64)] + [(o, 32) for o in mid] + [(len(orig) - 64, 64)]
+
+
+def main(ref):
     from oracle.oracle import xxh64
+    REF = os.path.join(ref, "ruzstd")
     man = {"source": "KillingSpark/zstd-rs eb7e03cc1b15705b94b93249ff7b05c4fc2c98b3", "corpus": {}, "dict": {}, "fixtures": {}, "fuzz": {}}
     # corpus
     dst = os.path.join(HERE, "decodecorpus"); os.makedirs(dst, exist_ok=True)
+    rng = np.random.Generator(np.random.PCG64(0xD0C0))
+    names, sizes, win_file, win_off, win_len, vals = [], [], [], [], [], []
     for f in sorted(os.listdir(f"{REF}/decodecorpus_files")):
         if not f.endswith(".zst"):
             continue
@@ -34,6 +47,12 @@ def main():
         orig = open(f"{REF}/decodecorpus_files/{f[:-4]}", "rb").read()
         man["corpus"][f] = {"size": len(orig), "sha256": sha(orig), "xxh64_low32": xxh64(orig) & 0xFFFFFFFF,
                             "compressed_size": os.path.getsize(f"{dst}/{f}")}
+        for o, n in original_windows(orig, rng):
+            win_file.append(len(names)); win_off.append(o); win_len.append(n); vals.append(np.frombuffer(orig[o:o + n], np.uint8))
+        names.append(f); sizes.append(len(orig))
+    np.savez_compressed(os.path.join(HERE, "decodecorpus_originals.npz"), name=np.array(names), size=np.array(sizes, np.uint64),
+                        win_file=np.array(win_file, np.uint32), win_off=np.array(win_off, np.uint64),
+                        win_len=np.array(win_len, np.uint32), val=np.concatenate(vals))
     # dict tests
     dst = os.path.join(HERE, "dict_tests", "files"); os.makedirs(dst, exist_ok=True)
     shutil.copyfile(f"{REF}/dict_tests/dictionary", os.path.join(HERE, "dict_tests", "dictionary"))
@@ -66,4 +85,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])
