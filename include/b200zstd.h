@@ -380,6 +380,50 @@ b200z_frame_decoder *b200z_streaming_decoder_frame_decoder(b200z_streaming_decod
 b200z_frame_decoder *b200z_streaming_decoder_into_frame_decoder(b200z_streaming_decoder *s);
 void b200z_streaming_decoder_free(b200z_streaming_decoder *s);
 
+/* ------------------------------------------------------------------------------------------------------------
+ * Compression -- ruzstd's encoding module (encoding/mod.rs, frame_compressor.rs:131-224) on the GPU.  Every 128 KiB block of
+ * every frame is compressed at once (the reference's Fastest matcher never looks outside the current block,
+ * match_generator.rs:28-53).  Frames: magic, no dictionary, not single-segment, Window_Descriptor 128 KiB
+ * (FrameHeader::serialize, frame_header.rs), blocks of at most 128 KiB, the last one empty when the input is a multiple of
+ * 128 KiB (frame_compressor.rs:141-186).  A frame's bytes depend only on its plaintext, the level and the flags.
+ * ---------------------------------------------------------------------------------------------------------- */
+/* CompressionLevel (encoding/mod.rs:47-68) */
+#define B200Z_LEVEL_UNCOMPRESSED 0   /* Raw blocks only: byte-identical to the reference                                  */
+#define B200Z_LEVEL_FASTEST 1        /* RLE / Compressed / Raw per block, as levels/fastest.rs decides                    */
+#define B200Z_LEVEL_DEFAULT 2        /* unimplemented!() in the reference (frame_compressor.rs:202-204):                 */
+#define B200Z_LEVEL_BETTER 3         /*   -> B200Z_ERR_REFERENCE_WOULD_PANIC                                              */
+#define B200Z_LEVEL_BEST 4
+#define B200Z_COMPRESS_CHECKSUM 1u     /* Content_Checksum (the reference's default, feature "hash")                       */
+#define B200Z_COMPRESS_CONTENT_SIZE 2u /* EXTENSION: write Frame_Content_Size (the reference writes none); the field is the
+                                          smallest of 2 / 4 / 8 bytes that holds it (the 1-byte field needs Single_Segment) */
+
+typedef struct b200z_compress_result {
+    uint64_t out_size;       /* compressed bytes written at out_off                                               */
+    int32_t status;          /* 0 or B200Z_ERR_TARGET_TOO_SMALL (out_cap, or the output buffer, is too short)    */
+    int32_t stage;
+    uint32_t num_blocks, raw_blocks, rle_blocks, compressed_blocks;
+    uint32_t checksum;       /* low 32 bits of XXH64(seed 0) of the plaintext, written when flagged             */
+    uint32_t reserved;
+} b200z_compress_result;
+
+/* largest frame b200z_compress_frames_batch writes for src_size bytes: header with Frame_Content_Size, 3 bytes per block,
+ * the plaintext (every block Raw) and the checksum */
+size_t b200z_compress_bound(size_t src_size);
+/* Many independent frames: frames[i] = {src_off, src_size, out_off, out_cap} (src = plaintext inside `input`, out = where
+ * the frame goes inside `output`); host or device memory on either side (B200Z_MEM_*).  Only results[i].out_size bytes at
+ * each successful frame's out_off are written; the rest of `output` is left as it was.  Returns 0 when the submission ran
+ * (per-frame outcome in results[i]), B200Z_ERR_REFERENCE_WOULD_PANIC for levels Default / Better / Best, or another
+ * b200z_error for a submission-level failure.
+ * Device memory: the whole submission is in flight at once, with a fixed worst-case scratch of about 570 KB per 128 KiB block
+ * at the Fastest level (about 4.4 x the plaintext), plus a device copy of host input and of host output.  There is no
+ * chunking: a submission that does not fit fails with B200Z_ERR_OUT_OF_MEMORY, and the caller splits it into several. */
+int b200z_compress_frames_batch(b200z_ctx *ctx, const uint8_t *input, size_t input_len, int input_mem, const b200z_frame_io *frames,
+                                size_t nframes, int level, uint32_t flags, uint8_t *output, size_t output_cap, int output_mem,
+                                b200z_compress_result *results);
+/* encoding::compress(source, target, level) (mod.rs:24-30): reads `read_cb` to EOF, writes one frame to `write_cb`
+ * (one submission: the device-memory limit above applies to the whole stream) */
+int b200z_compress(b200z_ctx *ctx, b200z_read_fn read_cb, void *ruser, b200z_write_fn write_cb, void *wuser, int level, uint32_t flags);
+
 /* XXH64(seed 0) of a host buffer -- the content-checksum hash the reference feeds on drain
  * (decode_buffer.rs:42,225,290,301); exposed so bindings can verify checksums like tests/decode_corpus.rs:61-74 */
 uint64_t b200z_xxh64(const uint8_t *data, size_t len);

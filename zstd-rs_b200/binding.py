@@ -26,6 +26,10 @@ ALL, UPTO_BLOCKS, UPTO_BYTES = 0, 1, 2
 MEM_HOST, MEM_DEVICE = 0, 1
 ERR_SKIP_FRAME = 8
 FLAG_CHECKSUM = 1
+ERR_REFERENCE_WOULD_PANIC = 200
+# CompressionLevel (encoding/mod.rs:47-68); Default / Better / Best are unimplemented!() in the reference
+LEVEL_UNCOMPRESSED, LEVEL_FASTEST, LEVEL_DEFAULT, LEVEL_BETTER, LEVEL_BEST = 0, 1, 2, 3, 4
+COMPRESS_CHECKSUM, COMPRESS_CONTENT_SIZE = 1, 2
 
 
 class FrameIO(C.Structure):
@@ -50,6 +54,8 @@ FRAME_RESULT_DTYPE = np.dtype([("out_size", "<u8"), ("bytes_read", "<u8"), ("con
                                ("status", "<i4"), ("stage", "<i4"), ("blocks_decoded", "<u4"), ("error_block", "<u4"),
                                ("has_checksum", "<u4"), ("checksum_from_data", "<u4"), ("has_dict_id", "<u4"), ("dict_id", "<u4"),
                                ("has_calculated_checksum", "<u4"), ("calculated_checksum", "<u4")])
+COMPRESS_RESULT_DTYPE = np.dtype([("out_size", "<u8"), ("status", "<i4"), ("stage", "<i4"), ("num_blocks", "<u4"), ("raw_blocks", "<u4"),
+                                  ("rle_blocks", "<u4"), ("compressed_blocks", "<u4"), ("checksum", "<u4"), ("reserved", "<u4")])
 assert FRAME_IO_DTYPE.itemsize == C.sizeof(FrameIO) and FRAME_RESULT_DTYPE.itemsize == C.sizeof(FrameResult)
 
 
@@ -143,6 +149,9 @@ def lib():
         "b200z_streaming_decoder_into_frame_decoder": (vp, [vp]),
         "b200z_streaming_decoder_free": (None, [vp]),
         "b200z_xxh64": (C.c_uint64, [vp, sz]),
+        "b200z_compress_bound": (sz, [sz]),
+        "b200z_compress_frames_batch": (C.c_int, [vp, vp, sz, C.c_int, vp, sz, C.c_int, C.c_uint32, vp, sz, C.c_int, vp]),
+        "b200z_compress": (C.c_int, [vp, READ_FN, vp, WRITE_FN, vp, C.c_int, C.c_uint32]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)          # AttributeError here == a symbol the header declares is not exported
@@ -344,6 +353,67 @@ def decode_frames(ctx, input, frames, output, dicts=None, forced_dict=None, max_
                                         res.ctypes.data)
     ctx._chk(e)
     return res
+
+
+def compress_bound(n):
+    """b200z_compress_bound: the largest frame compress_frames writes for n plaintext bytes."""
+    return lib().b200z_compress_bound(n)
+
+
+def _check_level(level):
+    if level in (LEVEL_DEFAULT, LEVEL_BETTER, LEVEL_BEST):   # frame_compressor.rs:202-204: unimplemented!()
+        raise B200ZError(ERR_REFERENCE_WOULD_PANIC, 0, f"compression level {level} is not implemented by the reference")
+    if level not in (LEVEL_UNCOMPRESSED, LEVEL_FASTEST):
+        raise ValueError(f"unknown compression level {level}")
+
+
+def _compress_flags(checksum, content_size):
+    return (COMPRESS_CHECKSUM if checksum else 0) | (COMPRESS_CONTENT_SIZE if content_size else 0)
+
+
+def compress_frames(ctx, input, frames, output, level=LEVEL_FASTEST, checksum=True, content_size=False):
+    """b200z_compress_frames_batch: many independent frames at once.  frames: FRAME_IO_DTYPE rows {src_off, src_size, out_off,
+    out_cap} (src = plaintext inside `input`, out = where the frame goes inside `output`); input/output: bytes, numpy or torch
+    (host or cuda).  Returns a COMPRESS_RESULT_DTYPE array."""
+    _check_level(level)
+    fr = _frames_array(frames)
+    res = np.zeros(len(fr), dtype=COMPRESS_RESULT_DTYPE)
+    ip, il, _k1 = _ptr(input)
+    op, ol, _k2 = _ptr(output)
+    e = ctx.L.b200z_compress_frames_batch(ctx.h, ip, il, MEM_DEVICE if _is_device(input) else MEM_HOST, fr.ctypes.data, len(fr), level,
+                                          _compress_flags(checksum, content_size), op, ol, MEM_DEVICE if _is_device(output) else MEM_HOST,
+                                          res.ctypes.data)
+    ctx._chk(e)
+    return res
+
+
+def compress(ctx, data, level=LEVEL_FASTEST, checksum=True, content_size=False):
+    """encoding::compress_to_vec (mod.rs:33-37): one frame for `data`, as bytes."""
+    _check_level(level)
+    src = bytes(data)
+    cap = compress_bound(len(src))
+    out = np.empty(cap, dtype=np.uint8)
+    io = np.array([(0, len(src), 0, cap)], dtype=FRAME_IO_DTYPE)
+    r = compress_frames(ctx, src, io, out, level, checksum, content_size)[0]
+    if r["status"]:
+        raise B200ZError(int(r["status"]), int(r["stage"]))
+    return out[:int(r["out_size"])].tobytes()
+
+
+def compress_stream(ctx, reader, writer, level=LEVEL_FASTEST, checksum=True, content_size=False):
+    """b200z_compress == encoding::compress(source, target, level) (mod.rs:24-30): reader.read(n) to EOF, writer.write(b)."""
+    _check_level(level)
+
+    def _rd(_user, buf, n):
+        b = reader.read(n)
+        if b:
+            C.memmove(buf, b, len(b))
+        return len(b)
+
+    def _wr(_user, buf, n):
+        return writer.write(C.string_at(buf, n)) or 0
+    rcb, wcb = READ_FN(_rd), WRITE_FN(_wr)
+    ctx._chk(ctx.L.b200z_compress(ctx.h, rcb, None, wcb, None, level, _compress_flags(checksum, content_size)))
 
 
 class Batch:

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/b200zstd.h"
+#include "compress.h"
 #include "kernels.h"
 #include "plan.h"
 #include "tables.cuh"
@@ -83,10 +84,12 @@ struct b200z_ctx {
     cudaStream_t side = nullptr;          // k_huf runs here, beside k_fse
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     struct PipeResources *pipe = nullptr;  // lazily created by the pipelined one-shot path
+    struct CompressResources *comp = nullptr;  // lazily created by the first compression call
     FseSlot *d_predef = nullptr;
     std::string err;
     uint64_t launches = 0;
     uint32_t flags = 0;
+    uint32_t match_ctas = 0;              // resident k_cmatch CTAs on this device (init_compress_kernels)
     int set_cuda_err(cudaError_t e, const char *what) {
         char buf[256];
         snprintf(buf, sizeof buf, "CUDA error in %s: %s", what, cudaGetErrorString(e));
@@ -119,7 +122,7 @@ extern "C" int b200z_ctx_create(int device, b200z_ctx **out) {
     if (cudaStreamCreateWithPriority(&c->side, cudaStreamNonBlocking, prio_lo) != cudaSuccess || cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); return B200Z_ERR_CUDA; }
     if (cudaMalloc((void **)&c->d_predef, sizeof(FseSlot)) != cudaSuccess) { cudaGetLastError(); return B200Z_ERR_OUT_OF_MEMORY; }
-    if (init_kernels()) { cudaGetLastError(); return B200Z_ERR_CUDA; }
+    if (init_kernels() || init_compress_kernels(&c->match_ctas)) { cudaGetLastError(); return B200Z_ERR_CUDA; }
     int e = launch_predefined(c->d_predef, c->stream);
     if (e || cudaStreamSynchronize(c->stream) != cudaSuccess) { cudaGetLastError(); return B200Z_ERR_CUDA; }
     c->launches = 1;
@@ -127,10 +130,12 @@ extern "C" int b200z_ctx_create(int device, b200z_ctx **out) {
     return 0;
 }
 static void pipe_free(b200z_ctx *c);
+static void comp_free(b200z_ctx *c);
 extern "C" void b200z_ctx_destroy(b200z_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
     pipe_free(c);
+    comp_free(c);
     if (c->d_predef) cudaFree(c->d_predef);
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_join) cudaEventDestroy(c->ev_join);
@@ -1640,4 +1645,118 @@ extern "C" void b200z_streaming_decoder_free(b200z_streaming_decoder *s) {
     if (!s) return;
     if (s->owns) b200z_frame_decoder_free(s->dec);
     delete s;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// compression (compress.cu): the plan is block counts and scratch offsets; scratch is a fixed worst case per block, kept in
+// the context and reused across calls.
+// ---------------------------------------------------------------------------------------------------------------
+struct CompressResources {
+    DevBuf d_in, d_out, d_frames, d_blocks, d_bout, d_block_off, d_hash, d_results, d_lits, d_seqs, d_body, d_cand;
+};
+static void comp_free(b200z_ctx *c) { delete c->comp; c->comp = nullptr; }
+
+extern "C" size_t b200z_compress_bound(size_t n) {
+    return 6 + enc_fcs_bytes(n) + 3 * (size_t)enc_num_blocks(n) + n + 4;
+}
+
+extern "C" int b200z_compress_frames_batch(b200z_ctx *c, const uint8_t *input, size_t input_len, int input_mem, const b200z_frame_io *frames,
+                                           size_t nframes, int level, uint32_t flags, uint8_t *output, size_t output_cap, int output_mem,
+                                           b200z_compress_result *results) {
+    if (level >= B200Z_LEVEL_DEFAULT && level <= B200Z_LEVEL_BEST) return B200Z_ERR_REFERENCE_WOULD_PANIC;   // unimplemented!()
+    if (level != B200Z_LEVEL_UNCOMPRESSED && level != B200Z_LEVEL_FASTEST) return B200Z_ERR_INVALID_ARGUMENT;
+    if (!c || (flags & ~(B200Z_COMPRESS_CHECKSUM | B200Z_COMPRESS_CONTENT_SIZE)) || (!results && nframes) || (!frames && nframes) ||
+        (!input && input_len) || (!output && output_cap))
+        return B200Z_ERR_INVALID_ARGUMENT;
+    if (int e = c->use()) return e;
+    if (!nframes) return 0;
+    std::vector<CFrame> hf(nframes);
+    std::vector<CBlock> hb;
+    uint64_t in_lo = UINT64_MAX, in_hi = 0;
+    for (size_t i = 0; i < nframes; i++) {
+        const b200z_frame_io &io = frames[i];
+        if (io.src_off > input_len || io.src_size > input_len - io.src_off) return B200Z_ERR_INVALID_ARGUMENT;
+        const uint64_t nb = enc_num_blocks(io.src_size);
+        if (hb.size() + nb > UINT32_MAX) return B200Z_ERR_INVALID_ARGUMENT;
+        hf[i] = CFrame{io.src_off, io.src_size, io.out_off, io.out_cap, (uint32_t)hb.size(), (uint32_t)nb};
+        for (uint64_t k = 0; k < nb; k++) {
+            const uint64_t off = k * ENC_BLOCK;
+            hb.push_back(CBlock{io.src_off + off, (uint32_t)std::min<uint64_t>(ENC_BLOCK, io.src_size - off), (uint32_t)i, (uint32_t)(k + 1 == nb), 0});
+        }
+        in_lo = std::min<uint64_t>(in_lo, io.src_off); in_hi = std::max<uint64_t>(in_hi, io.src_off + io.src_size);
+    }
+    if (!c->comp) c->comp = new CompressResources();
+    CompressResources &R = *c->comp;
+    const size_t nblocks = hb.size();
+    const uint32_t match_ctas = c->match_ctas;
+    int e = 0;
+    if ((e = R.d_frames.ensure(nframes * sizeof(CFrame))) || (e = R.d_blocks.ensure(nblocks * sizeof(CBlock))) ||
+        (e = R.d_bout.ensure(nblocks * sizeof(CBlockOut))) || (e = R.d_block_off.ensure(nblocks * 8)) || (e = R.d_hash.ensure(nframes * 8)) ||
+        (e = R.d_results.ensure(nframes * sizeof(b200z_compress_result))))
+        return e;
+    if (level == B200Z_LEVEL_FASTEST &&
+        ((e = R.d_lits.ensure(nblocks * (size_t)ENC_BLOCK)) || (e = R.d_seqs.ensure(nblocks * (size_t)ENC_MAX_SEQ * sizeof(EncSeq))) ||
+         (e = R.d_body.ensure(nblocks * (size_t)ENC_BODY_STRIDE)) || (e = R.d_cand.ensure((size_t)match_ctas * ENC_BLOCK * 4))))
+        return e;
+    const uint8_t *d_in = input;
+    if (input_mem != B200Z_MEM_DEVICE) {
+        if ((e = R.d_in.ensure(in_hi > in_lo ? in_hi - in_lo + 16 : 16))) return e;
+        if (in_hi > in_lo) CU(c, cudaMemcpyAsync(R.d_in.p, input + in_lo, in_hi - in_lo, cudaMemcpyHostToDevice, c->stream));
+        d_in = R.d_in.as<uint8_t>() - (in_hi > in_lo ? in_lo : 0);
+    }
+    uint8_t *d_out = output;
+    if (output_mem != B200Z_MEM_DEVICE) {
+        if ((e = R.d_out.ensure(output_cap + 16))) return e;
+        d_out = R.d_out.as<uint8_t>();
+    }
+    CU(c, cudaMemcpyAsync(R.d_frames.p, hf.data(), nframes * sizeof(CFrame), cudaMemcpyHostToDevice, c->stream));
+    CU(c, cudaMemcpyAsync(R.d_blocks.p, hb.data(), nblocks * sizeof(CBlock), cudaMemcpyHostToDevice, c->stream));
+    CompressArgs a{d_in, d_out, output_cap, R.d_frames.as<CFrame>(), R.d_blocks.as<CBlock>(), R.d_bout.as<CBlockOut>(), R.d_block_off.as<uint64_t>(),
+                   R.d_hash.as<uint64_t>(), R.d_results.as<b200z_compress_result>(), R.d_lits.as<uint8_t>(), R.d_seqs.as<EncSeq>(), R.d_body.as<uint8_t>(),
+                   R.d_cand.as<uint32_t>(), (uint32_t)nblocks, (uint32_t)nframes, (uint32_t)level, flags, match_ctas};
+    for (int k = 0; k < kCompressKernels; k++)
+        if (int le = launch_compress_stage(a, k, c->stream)) return c->set_cuda_err((cudaError_t)le, kCompressKernelNames[k]);
+    c->launches += compress_launch_count(a);
+    CU(c, cudaMemcpyAsync(results, R.d_results.p, nframes * sizeof(b200z_compress_result), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (output_mem != B200Z_MEM_DEVICE) {
+        // exactly the bytes each frame wrote: the caller's buffer between frames and under failed frames is left alone.  Frames
+        // that follow each other without a gap go back in one copy.
+        uint64_t lo = 0, hi = 0;
+        for (size_t i = 0; i <= nframes; i++) {
+            const bool wrote = i < nframes && results[i].status == 0 && results[i].out_size;
+            if (wrote && hi > lo && frames[i].out_off == hi) { hi += results[i].out_size; continue; }
+            if (hi > lo) CU(c, cudaMemcpyAsync(output + lo, d_out + lo, hi - lo, cudaMemcpyDeviceToHost, c->stream));
+            lo = hi = 0;
+            if (wrote) { lo = frames[i].out_off; hi = lo + results[i].out_size; }
+        }
+        CU(c, cudaStreamSynchronize(c->stream));
+    }
+    return 0;
+}
+
+extern "C" int b200z_compress(b200z_ctx *c, b200z_read_fn rd, void *ruser, b200z_write_fn wr, void *wuser, int level, uint32_t flags) {
+    if (level >= B200Z_LEVEL_DEFAULT && level <= B200Z_LEVEL_BEST) return B200Z_ERR_REFERENCE_WOULD_PANIC;
+    if (!c || !rd || !wr) return B200Z_ERR_INVALID_ARGUMENT;
+    std::vector<uint8_t> src;
+    for (;;) {   // read to EOF (frame_compressor.rs:151-163)
+        const size_t at = src.size();
+        src.resize(at + (1u << 20));
+        const long r = rd(ruser, src.data() + at, 1u << 20);
+        if (r < 0) { src.resize(at); c->err = "read callback failed"; return B200Z_ERR_INVALID_ARGUMENT; }
+        src.resize(at + (size_t)r);
+        if (r == 0) break;
+    }
+    const size_t cap = b200z_compress_bound(src.size());
+    std::vector<uint8_t> out(cap);
+    b200z_frame_io io{0, src.size(), 0, cap};
+    b200z_compress_result res{};
+    if (int e = b200z_compress_frames_batch(c, src.data(), src.size(), B200Z_MEM_HOST, &io, 1, level, flags, out.data(), cap, B200Z_MEM_HOST, &res)) return e;
+    if (res.status) return res.status;
+    for (size_t done = 0; done < res.out_size;) {   // write_all
+        const long w = wr(wuser, out.data() + done, (size_t)(res.out_size - done));
+        if (w <= 0) { c->err = "write callback failed"; return B200Z_ERR_INVALID_ARGUMENT; }
+        done += (size_t)w;
+    }
+    return 0;
 }
